@@ -43,7 +43,13 @@ def parse():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--quick", action="store_true", help="skip the auxiliary measurements (baseline / twins / e2e)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the ag_gemm and gemm_rs outputs of the last timed step as DIR/<name>.npy "
+                         "(float32; a fixed, seeded sample of rows; with several ranks one file per rank)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -123,6 +129,17 @@ def pin_numa_local(torch, device_index: int):
         return {"numa_node": node, "cpus": len(ids)}
     except Exception as e:      # noqa: BLE001
         return {"numa_node": None, "error": repr(e)[:80]}
+
+
+def dump_outputs(torch, out_dir, named, suffix=""):
+    """Write each output tensor of `named` ({name: (tensor, rows)}) as out_dir/<name><suffix>.npy in float32.  Only `rows` rows are
+    kept, chosen by a fixed seed, so the files stay small and two builds run with the same arguments compare row for row."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    g = torch.Generator().manual_seed(0)
+    for name, (t, rows) in named.items():
+        idx = torch.randperm(t.shape[0], generator=g)[:rows].sort().values.to(t.device)
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), t.index_select(0, idx).float().cpu().numpy())
 
 
 def link_gbs():
@@ -507,6 +524,11 @@ def main():
     ms_step = timed(step_ours, args.steps, max(3, args.warmup), sampler)
     launches = (_C.native_calls() - n0) * args.steps // (args.steps + max(3, args.warmup))
     clocks = sampler.stop() if me == 0 else None
+    if args.dump_outputs:
+        # ag_out / rs_out still hold the last timed step here; the measurements below overwrite them.  At most
+        # 512 x 4096 + 512 x 12288 floats (32 MiB) over all ranks.
+        dump_outputs(torch, args.dump_outputs, {"ag_gemm": (ag_out, 512), "gemm_rs": (rs_out, max(1, 512 // W))},
+                     "" if W == 1 else f"_rank{me}")
     flops_ag = 2.0 * AG["M"] * AG["N"] * AG["K"]
     flops_rs = 2.0 * RS["M"] * RS["N"] * RS["K"]
     tflops = (flops_ag + flops_rs) / (ms_step * 1e-3) / 1e12

@@ -13,9 +13,13 @@ def dist_env():
     # the emulation backend is forced only for the lifetime of this module's tests: setting it at import time would leak
     # into `pytest -m gpu` runs (pytest imports every test module during collection) and silently put GPU tests on the CPU
     import triton_dist.utils as U
+    # GPU tests earlier in the same session may have left the CUDA backend initialised; initialize_distributed would keep it,
+    # and the host-protocol tests below (a wait that must time out) would then wait on the device instead
+    U.finalize_distributed()
     os.environ.setdefault("MASTER_PORT", "29677")
     os.environ["TD_FORCE_HOST_BACKEND"] = "1"
     U.initialize_distributed(seed=0)
+    assert U.current_device().type == "cpu", "dist_env must run on the emulation backend"
     yield U
     U.finalize_distributed()
     os.environ.pop("TD_FORCE_HOST_BACKEND", None)
@@ -209,6 +213,26 @@ def test_bench_reference_arm_reports_unavailable():
     r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--gpus", "8"], capture_output=True, text=True,
                        timeout=120)
     assert r.returncode == 0 and "unavailable" in json.loads(r.stdout.strip().splitlines()[-1])
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs writes float32 .npy files holding the same seeded sample of rows on every run; --steps must be >= 1."""
+    import subprocess
+    import sys
+    import numpy as np
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+    t = torch.arange(64 * 3, dtype=torch.bfloat16).reshape(64, 3)
+    for d in ("a", "b"):
+        bench.dump_outputs(torch, str(tmp_path / d), {"x": (t, 8), "y": (t, 100)}, "_rank1")
+    a = np.load(tmp_path / "a" / "x_rank1.npy")
+    assert a.dtype == np.float32 and a.shape == (8, 3) and np.array_equal(a, np.load(tmp_path / "b" / "x_rank1.npy"))
+    rows = (a[:, 0] / 3).astype(np.int64)
+    assert (np.diff(rows) > 0).all() and np.array_equal(a, t.float().numpy()[rows])
+    assert np.array_equal(np.load(tmp_path / "a" / "y_rank1.npy"), t.float().numpy())
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and "--steps" in r.stderr
 
 
 def test_flash_attn_reference_paths():

@@ -53,19 +53,22 @@ def _digest(paths, extra: str) -> str:
 
 
 class _BuildLock:
-    """Inter-process lock: ranks launched together must not compile the same objects concurrently."""
+    """Inter-process lock: ranks launched together must not compile the same objects concurrently.
+
+    The lock file is opened read-only (flock needs no write access) and created only when missing, so that loading an
+    up-to-date build also works from a read-only checkout."""
 
     def __enter__(self):
         import fcntl
         LIBDIR.mkdir(parents=True, exist_ok=True)
-        self.f = open(LIBDIR / ".build.lock", "w")
-        fcntl.flock(self.f, fcntl.LOCK_EX)
+        self.fd = os.open(LIBDIR / ".build.lock", os.O_RDONLY | os.O_CREAT, 0o644)
+        fcntl.flock(self.fd, fcntl.LOCK_EX)
         return self
 
     def __exit__(self, *exc):
         import fcntl
-        fcntl.flock(self.f, fcntl.LOCK_UN)
-        self.f.close()
+        fcntl.flock(self.fd, fcntl.LOCK_UN)
+        os.close(self.fd)
 
 
 def _headers():
