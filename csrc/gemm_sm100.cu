@@ -47,6 +47,9 @@ struct TdGemmArgs {
   long long epd_topk, epd_epr, epd_cpd, epd_rows_cap; void* epd_meta; const void* c_route;
   const void* segk_off; long long segk_n;      // segmented-K batch (mode 0): C is [segk_n][M][N] (c_nbuf / c_buf_stride_bytes)
   const void* scale_a; const void* scale_b;    // fp32 per-row [M] / per-column [N] scales applied in the epilogue (8-bit kinds)
+  // AG with 8-bit A: scale_a is then my shard's per-row scale [ag_rows_per_rank]; for MXFP8, sfa / sfa_chunks are the symmetric
+  // scale-chunk workspace (both parity halves) and ag_sfa_local my shard's chunks
+  void* ag_scale_ws; const void* ag_sfa_local; long long ag_sfa_buf_chunks;
 };
 
 static int encode_tmap(CUtensorMap* out, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides_bytes,
@@ -184,8 +187,27 @@ TD_API int td_gemm_launch(const TdGemmArgs* a, void* stream_) {
   p.in_kind = a->is_bf16 == 3 ? 1 : a->is_bf16 == 4 ? 2 : 0;
   p.bk_elems = bk_elems;
   p.scale_a = reinterpret_cast<const float*>(a->scale_a); p.scale_b = reinterpret_cast<const float*>(a->scale_b);
-  if (q8 && (a->mode == kAG || a->mode == kMoeRS || a->mode == kEPD || a->mode == kEPC || a->a_gather)) {
-    drv::set_error("8-bit (int8 / e4m3 per-tensor) inputs: plain, gemm_rs and gemm_ar modes only"); return -1;
+  if (q8 && (a->mode == kMoeRS || a->mode == kEPD || a->mode == kEPC || a->a_gather)) {
+    drv::set_error("8-bit (int8 / e4m3 per-tensor) inputs: plain, ag_gemm, gemm_rs and gemm_ar modes only"); return -1;
+  }
+  p.ag_esz = esz;
+  if (a->mode == kAG && (q8 || fp8) && a->world > 1) {
+    if (a->ag_copy_local == 2 || a->ag_skip_wait == 2) {
+      drv::set_error("ag_gemm: 8-bit inputs take the in-kernel transports (sm_k / multicast / sm), not copy_engine or all-to-all"); return -1;
+    }
+    if (a->ag_copy_local != 1 || !a->ag_a_local) { drv::set_error("ag_gemm: 8-bit inputs are pushed from the caller's shard (ag_a_local)"); return -1; }
+    if (q8 && a->scale_a && !a->ag_scale_ws) { drv::set_error("ag_gemm: per-row scales of 8-bit A need the scale workspace"); return -1; }
+    if (fp8) {
+      if (a->ag_rows_per_rank % BM != 0) { drv::set_error("ag_gemm: MXFP8 needs (M / world) %% 128 == 0 (one scale chunk covers 128 rows)"); return -1; }
+      if (!a->ag_sfa_local || a->ag_sfa_buf_chunks * 2 != a->sfa_chunks ||
+          a->ag_sfa_buf_chunks * BM < (a->ag_ws_buf_bytes / a->K) * (long long)p.num_k) {
+        drv::set_error("ag_gemm: MXFP8 needs the scale-chunk workspace [2][max_M / 128][K / 128][512] and the shard's chunks"); return -1;
+      }
+    }
+    p.ag_scale_ws = q8 ? reinterpret_cast<float*>(a->ag_scale_ws) : nullptr;
+    p.ag_sf_ws = fp8 ? reinterpret_cast<char*>(const_cast<void*>(a->sfa)) : nullptr;
+    p.ag_sf_local = fp8 ? reinterpret_cast<const char*>(a->ag_sfa_local) : nullptr;
+    p.ag_sf_buf_chunks = fp8 ? a->ag_sfa_buf_chunks : 0;
   }
   p.n_comm_ctas = (int)a->n_comm_ctas;
   p.C = a->C; p.ldc = a->ldc;
@@ -224,7 +246,7 @@ TD_API int td_gemm_launch(const TdGemmArgs* a, void* stream_) {
     const bool mcast = a->ag_skip_wait == 3;
     if (mcast && !a->mc_base) { drv::set_error("ag_gemm: multicast transport needs an NVLS multicast mapping"); return -1; }
     if (a->ag_copy_local == 2) { drv::set_error("ag_gemm: the all-to-all flavour cannot use the K-sliced transports"); return -1; }
-    if (a->a_gather || fp8) { drv::set_error("ag_gemm: the K-sliced transports take dense 16-bit A"); return -1; }
+    if (a->a_gather) { drv::set_error("ag_gemm: the K-sliced transports take dense A"); return -1; }
     if (a->ag_rows_per_rank % BM != 0) { drv::set_error("ag_gemm: K-sliced transports need (M / world) %% 128 == 0"); return -1; }
     if (!mcast && !a->ag_a_local) { drv::set_error("ag_gemm: the P2P K-sliced transport reads the caller's shard (ag_a_local)"); return -1; }
     if (p.n_comm_ctas < cg) p.n_comm_ctas = mcast ? 24 : 32;
@@ -270,7 +292,7 @@ TD_API int td_gemm_launch(const TdGemmArgs* a, void* stream_) {
     while (nsub > 1 && (p.n_comm_ctas * nsub > kAGMaxSlices || shard / (p.n_comm_ctas * nsub) < (64u << 10))) nsub >>= 1;
     p.ag_nslices = p.n_comm_ctas * nsub;
   }
-  if (a->mode == kAG && !fp8 && !a->a_gather && a->ag_skip_wait != 2 && a->ag_copy_local != 0 && a->ag_a_local &&
+  if (a->mode == kAG && !a->a_gather && a->ag_skip_wait != 2 && a->ag_copy_local != 0 && a->ag_a_local &&
       a->ag_rows_per_rank % BM == 0) {
     // tiles of the local rows are loaded straight from the caller's shard: {K, local rows}, same 64 x 128 box
     const long long lrows = a->ag_copy_local == 2 ? a->ag_rows_per_rank * a->world : a->ag_rows_per_rank;
@@ -278,6 +300,13 @@ TD_API int td_gemm_launch(const TdGemmArgs* a, void* stream_) {
     cuuint64_t strides[1] = {(cuuint64_t)a->K * esz};
     cuuint32_t box[2] = {(cuuint32_t)bk_elems, BM};
     if (encode_tmap(&p.tmap_al, a->ag_a_local, 2, dims, strides, box, bf16)) return -1;
+    if (fp8) {   // and their scale chunks from the caller's tensor: the workspace copy is filled by peers during this launch
+      if (!a->ag_sfa_local) { drv::set_error("ag_gemm: MXFP8 needs the shard's scale chunks"); return -1; }
+      cuuint64_t ds[2] = {128, (cuuint64_t)(a->ag_rows_per_rank / BM * p.num_k)};
+      cuuint64_t st[1] = {512};
+      cuuint32_t bx[2] = {128, 1};
+      if (encode_tmap(&p.tmap_sfal, a->ag_sfa_local, 2, ds, st, bx, 3)) return -1;
+    }
     p.ag_local_direct = 1;
   }
   p.rs_skip_wait = (int)a->rs_skip_wait; p.rs_fp32 = (int)a->rs_fp32;

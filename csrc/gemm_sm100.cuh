@@ -124,6 +124,14 @@ struct Params {
   long long ag_ws_buf_bytes; // bytes of one buffer
   uint32_t* ag_flags;        // symmetric: [2][world(src)][kAGMaxSlices] = phase of the call that pushed that slice
   uint32_t* ag_ready;        // [world]: ag_ready[s] >= p  <=>  rank s has its phase-p shard in ITS workspace (symmetric)
+  int ag_esz;                // bytes per element of A: 2 (16-bit) or 1 (int8 / e4m3 / MXFP8); a gathered row is K * ag_esz bytes
+  int pad4;
+  // 8-bit payload that travels with the rows (see ag_push_scales).  scale_a is then MY shard's per-row scale [rows_per_rank]
+  float* ag_scale_ws;        // int8 / e4m3: symmetric fp32 [2][rows of one workspace half], gathered per-row activation scales
+  char* ag_sf_ws;            // MXFP8: symmetric UE8M0 chunks [2][ag_sf_buf_chunks][512]; tmap_sfa spans both halves
+  const char* ag_sf_local;   // MXFP8: my shard's chunks [rows_per_rank / 128][num_k][512] (the caller's tensor, also tmap_sfal)
+  long long ag_sf_buf_chunks;
+  CUtensorMap tmap_sfal;     // MXFP8, own rows read directly (ag_local_direct): {128 (uint32), chunks of my shard}
   // ---- RS (ring) ----
   int rs_rows_per_rank;      // M / world, multiple of BM * cta_group
   int rs_skip_wait;          // GEMM-only twin: never wait for the partial of rank+1 (adds whatever the staging holds)
@@ -260,7 +268,7 @@ TD_DEVICE void ag_wait_rows(const Params& p, uint32_t ph, int row0, int row1) {
   // destination.  A flag holds the phase number of the call that last filled it, so stale values from earlier
   // calls (or other shapes) are simply "< ph" and nothing is ever reset.
   const int Ms = p.ag_rows_per_rank;
-  const size_t row_bytes = static_cast<size_t>(p.K) * 2;
+  const size_t row_bytes = static_cast<size_t>(p.K) * p.ag_esz;
   const size_t shard_bytes = static_cast<size_t>(Ms) * row_bytes;
   const size_t slice = ag_slice_bytes(shard_bytes, p.ag_nslices);
   const uint32_t* flags = p.ag_flags + (ph & 1u) * p.symm.world * kAGMaxSlices;
@@ -300,9 +308,35 @@ TD_DEVICE void ag_wait_kslice(const Params& p, uint32_t ph, int s, int r_local, 
 // following cp.async.bulk completion was observed to overtake the data), and that fence is expensive while
 // the SM has NVLink writes in flight -- so it is issued once per (CTA, destination), after a whole slice.
 // -------------------------------------------------------------------------------------------------
+// 8-bit kinds: the scales that belong to rows [r0, r1) of my shard, stored by all threads of a comm CTA into rank d's workspace
+// half par, BEFORE the release fence that publishes the rows (so the rows' flag covers them; there are no extra flags):
+//  * per-row activation scales (int8 / e4m3; with_rows): scale_a[r] -> ag_scale_ws[par][me * Ms + r].  A per-tensor scale was
+//    expanded to my rows by the caller, so every source's rows carry their own rank's scale.
+//  * MXFP8: the 512-byte chunks of k-blocks [kb0, kb1) of every 128-row block whose FIRST row lies in [r0, r1).  That block's
+//    first row is pushed by this CTA, so a consumer waiting for the first row's flag (ag_wait_rows / ag_wait_kslice) has the chunk.
+TD_DEVICE void ag_push_scales(const Params& p, uint32_t par, int d, int r0, int r1, int kb0, int kb1, bool with_rows) {
+  const int me = p.symm.rank, Ms = p.ag_rows_per_rank;
+  if (with_rows && p.ag_scale_ws != nullptr) {
+    const size_t rows_buf = p.ag_ws_buf_bytes / (static_cast<size_t>(p.K) * p.ag_esz);
+    float* dst = symm_at(p.symm, p.ag_scale_ws + par * rows_buf + static_cast<size_t>(me) * Ms, d);
+    for (int r = r0 + static_cast<int>(threadIdx.x); r < r1; r += kThreads) dst[r] = p.scale_a[r];
+  }
+  if (p.ag_sf_ws != nullptr) {
+    const int b0 = (r0 + BM - 1) / BM, b1 = (r1 + BM - 1) / BM, nkb = kb1 - kb0;
+    constexpr int kPieces = kSFChunk / 16;
+    const int n = max(0, b1 - b0) * max(0, nkb) * kPieces;
+    char* dst = symm_at(p.symm, p.ag_sf_ws + (static_cast<size_t>(par) * p.ag_sf_buf_chunks + static_cast<size_t>(me) * (Ms / BM) * p.num_k) * kSFChunk, d);
+    for (int i = threadIdx.x; i < n; i += kThreads) {
+      const int c = i / kPieces;
+      const size_t off = (static_cast<size_t>(b0 + c / nkb) * p.num_k + kb0 + c % nkb) * kSFChunk + (i % kPieces) * 16;
+      ptx::st_na_v4(dst + off, ptx::ld_nc_v4(p.ag_sf_local + off));
+    }
+  }
+}
+
 TD_DEVICE void ag_comm_cta(const Params& p, uint32_t ph, int comm_idx) {
   const int W = p.symm.world, me = p.symm.rank, Ms = p.ag_rows_per_rank;
-  const size_t row_bytes = static_cast<size_t>(p.K) * 2;
+  const size_t row_bytes = static_cast<size_t>(p.K) * p.ag_esz;
   const size_t shard_bytes = static_cast<size_t>(Ms) * row_bytes;
   const size_t slice = ag_slice_bytes(shard_bytes, p.ag_nslices);
   char* ws = p.ag_ws + (ph & 1u) * p.ag_ws_buf_bytes;
@@ -359,6 +393,9 @@ TD_DEVICE void ag_comm_cta(const Params& p, uint32_t ph, int comm_idx) {
           }
         }
       }
+      if (p.ag_scale_ws != nullptr || p.ag_sf_ws != nullptr)   // scales of my rows with slice 0, MXFP8 chunks of slice j's k-blocks
+        for (int d = (p.ag_multicast || !p.ag_local_direct) ? 0 : 1; d < W; ++d)
+          ag_push_scales(p, ph & 1u, (me + d) % W, r0, r1, p.ag_slice_kb[j], p.ag_slice_kb[j + 1], j == 0);
       __syncthreads();
       if (threadIdx.x == 0) {
         prof_record(p.prof, pslot, 1, false);
@@ -379,6 +416,9 @@ TD_DEVICE void ag_comm_cta(const Params& p, uint32_t ph, int comm_idx) {
       const size_t b0 = min(shard_bytes, slice * sidx), b1 = min(shard_bytes, b0 + slice);
       if (threadIdx.x == 0) prof_record(p.prof, pslot, 1, true);
       if (b1 > b0) copy16_strided_deep(symm_at(p.symm, ws, d) + shard_off + b0, src0 + a2a_off + b0, b1 - b0, threadIdx.x, kThreads);
+      if (p.ag_scale_ws != nullptr || p.ag_sf_ws != nullptr)   // rows whose first byte is in this slice
+        ag_push_scales(p, ph & 1u, d, static_cast<int>((b0 + row_bytes - 1) / row_bytes), static_cast<int>((b1 + row_bytes - 1) / row_bytes),
+                       0, p.num_k, true);
       __syncthreads();
       if (threadIdx.x == 0) {
         prof_record(p.prof, pslot, 1, false);
@@ -717,7 +757,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_kernel(const __grid_constant
             // slices (source rank, comm CTA) that carry ITS four rows, then the rows are gathered by TMA
             const int rr[4] = {r0, r1, r2, r3};
             const int Ms = p.ag_rows_per_rank;
-            const size_t row_bytes = static_cast<size_t>(p.K) * 2;
+            const size_t row_bytes = static_cast<size_t>(p.K) * p.ag_esz;
             const size_t slice = ag_slice_bytes(static_cast<size_t>(Ms) * row_bytes, p.ag_nslices);
             const uint32_t* flags = p.ag_flags + (ph & 1u) * p.symm.world * kAGMaxSlices;
             if (!p.ag_skip_wait) {
@@ -808,7 +848,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_kernel(const __grid_constant
               else ptx::tma_load_3d(&p.tmap_a, full_bar + stage, sa, kb * kBKElems, row0, abuf);
               ptx::tma_load_2d(&p.tmap_b, full_bar + stage, sb, kb * kBKElems, brow0, ptx::kEvictLast);
               if constexpr (kFP8) {
-                ptx::tma_load_2d(&p.tmap_sfa, full_bar + stage, ssfa, 0, (row0 / 128) * p.num_k + kb);
+                if (a_local) ptx::tma_load_2d(&p.tmap_sfal, full_bar + stage, ssfa, 0, (lrow0 / 128) * p.num_k + kb);
+                else ptx::tma_load_2d(&p.tmap_sfa, full_bar + stage, ssfa, 0, (row0 / 128) * p.num_k + kb + abuf * static_cast<int>(p.ag_sf_buf_chunks));
 #pragma unroll
                 for (int g = 0; g < (BN + 127) / 128; ++g)
                   ptx::tma_load_2d(&p.tmap_sfb, full_bar + stage, ssfb + g * kSFChunk, 0, ((n_tile * BN) / 128 + g) * p.num_k + kb);
@@ -821,7 +862,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_kernel(const __grid_constant
               else ptx::tma_load_3d_2sm(&p.tmap_a, full_bar + stage, sa, kb * kBKElems, row0, abuf);
               ptx::tma_load_2d_2sm(&p.tmap_b, full_bar + stage, sb, kb * kBKElems, brow0, ptx::kEvictLast);
               if constexpr (kFP8) {
-                ptx::tma_load_2d_2sm(&p.tmap_sfa, full_bar + stage, ssfa, 0, (row0 / 128) * p.num_k + kb);
+                if (a_local) ptx::tma_load_2d_2sm(&p.tmap_sfal, full_bar + stage, ssfa, 0, (lrow0 / 128) * p.num_k + kb);
+                else ptx::tma_load_2d_2sm(&p.tmap_sfa, full_bar + stage, ssfa, 0, (row0 / 128) * p.num_k + kb + abuf * static_cast<int>(p.ag_sf_buf_chunks));
 #pragma unroll
                 for (int g = 0; g < (BN + 127) / 128; ++g)
                   ptx::tma_load_2d_2sm(&p.tmap_sfb, full_bar + stage, ssfb + g * kSFChunk, 0, ((n_tile * BN) / 128 + g) * p.num_k + kb);
@@ -1022,6 +1064,31 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_kernel(const __grid_constant
           }
           ptx::named_bar_sync(2, kEpiThreads);
         } else if constexpr (kMode == kRS) { if (rs_step > 0) ptx::named_bar_sync(2, kEpiThreads); }  // flag acquired by et==0
+        // kAG, int8 / e4m3: the per-row scale of a gathered row.  Own rows read the caller's scale_a (never written during the
+        // launch).  A peer's scale was stored into ag_scale_ws by the comm CTA that pushed the row, before the release fence of
+        // that row's flag (ag_push_scales).  The TMA producer acquired the flag, but the only path from that acquire to these
+        // plain loads runs through TMA completion, tcgen05.mma and tcgen05.commit, which the memory model does not spell out as
+        // a release / acquire chain.  So one thread re-acquires the flags of the tile's rows (already raised: one load each)
+        // and the named barrier orders the other epilogue threads' loads after that acquire, as for the RS partials above.
+        float ag_row_sa = 1.f;
+        if constexpr (kMode == kAG) {
+          if (p.ag_scale_ws != nullptr && row_base < p.M) {
+            const int Ms = p.ag_rows_per_rank, s0 = row_base / Ms;
+            if (!p.ag_skip_wait) {
+              if (et == 0) {
+                if (!p.ag_kslices) ag_wait_rows(p, ph, row_base, min(p.M, row_base + BM));
+                else if (s0 != p.symm.rank) ag_wait_kslice(p, ph, s0, row_base - s0 * Ms, 0);
+              }
+              ptx::named_bar_sync(2, kEpiThreads);
+            }
+            const int grow = row_base + my_row;
+            if (grow < p.M) {
+              const int s = grow / Ms;
+              const size_t rows_buf = p.ag_ws_buf_bytes / (static_cast<size_t>(p.K) * p.ag_esz);
+              ag_row_sa = s == p.symm.rank ? p.scale_a[grow - s * Ms] : p.ag_scale_ws[(ph & 1u) * rows_buf + grow];
+            }
+          }
+        }
 
 #pragma unroll 1
         for (int cb = 0; cb < kNumCBlocks; ++cb) {
@@ -1050,7 +1117,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_kernel(const __grid_constant
             }
             if (p.scale_a != nullptr || p.scale_b != nullptr) {       // dequantise: C = acc * scale_a[row] * scale_b[col]
               const int grow = row_base + my_row, gcol = col_base + cb * kCBlockCols + h * 32;
-              const float sa = (p.scale_a != nullptr && grow < p.M) ? p.scale_a[grow] : 1.f;
+              const float sa = (kMode == kAG && p.ag_scale_ws != nullptr) ? ag_row_sa
+                               : (p.scale_a != nullptr && grow < p.M) ? p.scale_a[grow] : 1.f;
 #pragma unroll
               for (int i = 0; i < 32; ++i) f[i] *= sa * ((p.scale_b != nullptr && gcol + i < p.N) ? p.scale_b[gcol + i] : 1.f);
             }

@@ -67,6 +67,7 @@ class GemmArgs(C.Structure):
         ("epd_send_off", c_void_p), ("epd_send_ids", c_void_p), ("epd_dest_off", c_void_p), ("epd_x", c_void_p),
         ("epd_topk", c_ll), ("epd_epr", c_ll), ("epd_cpd", c_ll), ("epd_rows_cap", c_ll), ("epd_meta", c_void_p), ("c_route", c_void_p),
         ("segk_off", c_void_p), ("segk_n", c_ll), ("scale_a", c_void_p), ("scale_b", c_void_p),
+        ("ag_scale_ws", c_void_p), ("ag_sfa_local", c_void_p), ("ag_sfa_buf_chunks", c_ll),
     ]]
 
 

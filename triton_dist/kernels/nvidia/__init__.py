@@ -1,6 +1,6 @@
 """``triton_dist.kernels.nvidia`` -- the reference's op namespace (kernels/nvidia/__init__.py:25-101), re-exported
 from :mod:`triton_dist.ops` where the sm_100a implementations live."""
-from ...ops.ag_gemm import (AllGatherGEMMTensorParallelContext, ag_gemm, create_ag_gemm_context, gemm_non_persistent,  # noqa: F401
+from ...ops.ag_gemm import (AllGatherGEMMTensorParallelContext, ag_gemm, ag_gemm_mxfp8, create_ag_gemm_context, gemm_non_persistent,  # noqa: F401
                             gemm_persistent)
 from ...ops.allgather import (AllGatherMethod, cp_engine_producer_all_gather_inter_node,  # noqa: F401
                               cp_engine_producer_all_gather_intra_node, get_auto_all_gather_method)

@@ -14,11 +14,12 @@ import torch.distributed as dist
 
 from .. import utils as U
 from ..ops import comm
-from ..ops.ag_gemm import ag_gemm, create_ag_gemm_context
+from ..ops.ag_gemm import ag_gemm, ag_gemm_mxfp8, create_ag_gemm_context
 from ..ops.elementwise import silu_mul
 from ..ops.gemm import gemm
 from ..ops.gemm_ar import create_gemm_ar_context_auto, low_latency_gemm_allreduce_op
-from ..ops.gemm_rs import create_gemm_rs_context, gemm_rs
+from ..ops.fp8 import quantize_mxfp8
+from ..ops.gemm_rs import create_gemm_rs_context, gemm_rs, gemm_rs_mxfp8
 
 
 def shard_local(tensor: torch.Tensor, world_size: int, dim: int, local_rank: int) -> torch.Tensor:
@@ -41,6 +42,7 @@ class TP_MLP:
         self.down_proj: Optional[torch.Tensor] = None      # [H, I / W]
         self.ag_ctx = self.rs_ctx = self.ar_ctx = self.gemm_ar_ctx = None
         self.ar_method = comm.AllReduceMethod.Unknown
+        self.gate_up_mx = self.down_mx = None               # MXFP8 weights of dist_triton_mxfp8_fwd
 
     # ---- parameters -------------------------------------------------------------------------------------
     def _init_parameters(self, mlp, verbose: bool = False):
@@ -62,9 +64,16 @@ class TP_MLP:
         self.dtype = self.gate_up_proj.dtype
 
     # ---- contexts -----------------------------------------------------------------------------------------
-    def _init_ctx(self, max_M: int, ag_intranode_stream=None, ag_internode_stream=None):
-        self.ag_ctx = create_ag_gemm_context(max_M, self.ag_N_per_rank, self.K, self.dtype, self.rank, self.world_size)
-        self.rs_ctx = create_gemm_rs_context(max_M, self.K, self.rank, self.world_size, self.world_size, self.dtype)
+    def _init_ctx(self, max_M: int, ag_intranode_stream=None, ag_internode_stream=None, mxfp8: bool = False):
+        """``mxfp8=True``: contexts for :meth:`dist_triton_mxfp8_fwd` (e4m3 all-gather workspace with its block scales) and the
+        gate/up and down weights quantised to MXFP8 once, here; :meth:`dist_triton_fwd` then needs a context of its own."""
+        ag_dtype = torch.float8_e4m3fn if mxfp8 else self.dtype
+        self.ag_ctx = create_ag_gemm_context(max_M, self.ag_N_per_rank, self.K, ag_dtype, self.rank, self.world_size)
+        self.rs_ctx = create_gemm_rs_context(max_M, self.K, self.rank, self.world_size, self.world_size,
+                                             torch.bfloat16 if mxfp8 else self.dtype)
+        if mxfp8:
+            self.gate_up_mx = quantize_mxfp8(self.gate_up_proj)
+            self.down_mx = quantize_mxfp8(self.down_proj)
         U.barrier_all_host()
 
     def _init_AR_ctx(self, max_M: int, method=comm.AllReduceMethod.Unknown, dtype=torch.bfloat16):
@@ -101,6 +110,19 @@ class TP_MLP:
         h = ag_gemm(x2, self.gate_up_proj.t(), self.ag_ctx)
         h = silu_mul(h)
         out = gemm_rs(h, self.down_proj.t(), self.rs_ctx)
+        return out.view(*shp[:-1], -1) if len(shp) == 3 else out
+
+    @torch.inference_mode()
+    def dist_triton_mxfp8_fwd(self, x: torch.Tensor) -> torch.Tensor:
+        """MXFP8 TP MLP (contexts from ``_init_ctx(..., mxfp8=True)``): quantise x -> AG-GEMM on e4m3 rows + block scales ->
+        fused SiLU*up -> quantise -> GEMM-RS, bf16 out.  ``x``: this rank's rows ``[M/W, H]`` (``M/W % 128 == 0``)."""
+        if self.gate_up_mx is None:
+            raise RuntimeError("dist_triton_mxfp8_fwd needs _init_ctx(max_M, mxfp8=True)")
+        shp = x.shape
+        x2 = x.reshape(-1, shp[-1])
+        h = ag_gemm_mxfp8(quantize_mxfp8(x2), self.gate_up_mx, self.ag_ctx)
+        h = silu_mul(h)
+        out = gemm_rs_mxfp8(quantize_mxfp8(h), self.down_mx, self.rs_ctx)
         return out.view(*shp[:-1], -1) if len(shp) == 3 else out
 
     @torch.inference_mode()
